@@ -161,6 +161,25 @@ class ClockSampler:
                 "source": source}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, per_frame):
+    """What the last timed step returns to a caller (PoseEngine.fetch_arrays): humans.npy, every person row
+    [k, 73] (score, 18 x (x, y, peak score, peak id | -1)) of every frame in frame order, and humans_per_frame.npy.
+    Above DUMP_BYTES the rows are a fixed seeded sample, and humans_index.npy names the rows kept."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = np.array([len(r) for r in per_frame], np.float64)
+    rows = np.concatenate(per_frame).astype(np.float32)
+    cap = (DUMP_BYTES - counts.nbytes) // (rows.shape[1] * rows.itemsize)
+    if len(rows) > cap:
+        keep = np.sort(np.random.RandomState(0).choice(len(rows), cap, replace=False))
+        rows = rows[keep]
+        np.save(os.path.join(out_dir, "humans_index.npy"), keep.astype(np.float64))
+    np.save(os.path.join(out_dir, "humans.npy"), rows)
+    np.save(os.path.join(out_dir, "humans_per_frame.npy"), counts)
+
+
 def synthetic_weights():
     import _b200_alias
     return importlib.import_module(_b200_alias.PKG + ".synthetic").he_state_arrays(1234)
@@ -271,6 +290,8 @@ def run_ours(args):
     ms_dev = e0.elapsed_time(e1)
     launches = nat.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.fetch_arrays(check=False))
     barrier()
 
     # ---- end-to-end timing through the public API with host buffers (e2e): every step copies its uint8 frames from
@@ -502,7 +523,14 @@ def main():
                     help="multi-scale test-time averaging around 368 (BASELINE.json configs[4]: 0.5,1.0,1.5,2.0 with --flip --batch 8)")
     ap.add_argument("--raw", type=int, default=0, metavar="N",
                     help="feed N x N raw frames and run crop_with_factor (resize to 368 x 368) on the device as well")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the persons the last step found (rank 0) to DIR/*.npy; the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3)
     global BATCH
     BATCH = args.batch

@@ -158,3 +158,16 @@ def fuzz_persons(rs, h, w):
             if k2 != k and (k, pa) in pts and (k2, pb) in pts and rs.rand() < 0.35:
                 draw(pts[(k, pa)], pts[(k2, pb)], _PAFCH[l][0], _PAFCH[l][1], float(rs.choice([0.5, 0.8, 1.0])))
     return jl, np.ascontiguousarray(paf)
+
+
+def fuzz_scenario(t):
+    """Scenario t of the pafprocess fuzz tests: (h, w, joint list, paf [h,w,38]); odd t person-shaped, even t random
+    fields (uniform / cluster / ties in turn)."""
+    rs = np.random.RandomState(1000 + t)
+    h, w = int(rs.choice([12, 23, 46])), int(rs.choice([23, 46, 53]))
+    if t % 2:
+        h = max(h, 23)
+        jl, paf = fuzz_persons(rs, h, w)
+    else:
+        jl, paf = fuzz_field(rs, h, w, ("uniform", "cluster", "ties")[(t // 2) % 3])
+    return h, w, jl, paf

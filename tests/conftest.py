@@ -1,3 +1,4 @@
+import hashlib
 import importlib
 import os
 import sys
@@ -46,6 +47,46 @@ POST_CASES = {
     "empty": lambda s: (np.zeros((46, 46, 19), np.float32), np.zeros((46, 46, 38), np.float32)),
     "p5_40x52": lambda s: s.stick_figures(5, 55, h=40, w=52)[:2],
 }
+
+
+class RecordedPafprocess:
+    """The getters of the reference's own pafprocess.cpp (the SWIG module's surface) as it answered on the scenarios of
+    oracle/synth.fuzz_scenario (golden pafprocess_ref, written by tests/golden/make_golden.py)."""
+
+    def __init__(self):
+        g = golden("pafprocess_ref")
+        self._digest, self._count = g["fuzz_digest"], g["fuzz_humans"]
+        self._score, self._cid, self._part = g["fuzz_score"], g["fuzz_cid"], g["fuzz_part"]
+        self._start = np.concatenate([[0], np.cumsum(np.maximum(self._count, 0))])
+
+    def select(self, t, jl, paf):
+        """Stands for process_paf on scenario t; jl / paf must be the inputs the recording was made from."""
+        h = hashlib.sha256()
+        for a in (jl, paf):
+            h.update(np.ascontiguousarray(a).tobytes())
+        assert h.hexdigest()[:16] == str(self._digest[t]), "scenario %d differs from the recorded input" % t
+        assert self._count[t] >= 0, "scenario %d was not recorded" % t
+        self._lo, self._n = int(self._start[t]), int(self._count[t])
+        self._peaks = {int(c): tuple(self._part[self._lo + hid, p]) for hid in range(self._n) for p, c in
+                       enumerate(self._cid[self._lo + hid]) if c >= 0}
+
+    def get_num_humans(self):
+        return self._n
+
+    def get_score(self, hid):
+        return float(self._score[self._lo + hid])
+
+    def get_part_cid(self, hid, part):
+        return int(self._cid[self._lo + hid, part])
+
+    def get_part_x(self, cid):
+        return int(self._peaks[cid][0])
+
+    def get_part_y(self, cid):
+        return int(self._peaks[cid][1])
+
+    def get_part_score(self, cid):
+        return float(np.float32(self._peaks[cid][2]))
 
 
 def humans_rows_to_dicts(rows):

@@ -14,7 +14,7 @@ import os
 import sys
 import types
 
-ARGS = sys.argv[1:]     # optional: "crop" / "eval" / "pre" regenerate only those small fixtures
+ARGS = sys.argv[1:]     # optional: "crop" / "eval" / "pre" / "paf" / "scripts" regenerate only those small fixtures
 
 import numpy as np
 
@@ -146,8 +146,92 @@ def make_preprocess():
     print("preprocess fixture written")
 
 
+def post_cases():
+    return [("p1", synth.stick_figures(1, 1)[:2]), ("p3", synth.stick_figures(3, 3)[:2]),
+            ("p8", synth.stick_figures(8, 8)[:2]), ("p30", synth.stick_figures(30, 30)[:2]),
+            ("noise0", synth.noise_maps(0)), ("empty", (np.zeros((46, 46, 19), np.float32), np.zeros((46, 46, 38), np.float32))),
+            ("p5_40x52", synth.stick_figures(5, 55, h=40, w=52)[:2])]
+
+
+FUZZ_SCENARIOS = 300
+TIES_CASES = ((30, 31), (50, 5), (80, 7))
+
+
+def make_pafprocess():
+    """The reference's own pafprocess.cpp (oracle/_ref, compiled as-is) on the inputs the tests feed it:
+      * fuzz_*: the getters after process_paf on synth.fuzz_scenario(t), t < FUZZ_SCENARIOS (heat_up all zero, paf
+        upsampled x8 by repetition); fuzz_humans[t] = -1 marks a scenario without peaks (never run);
+      * post_<case> / ties_<persons>_<seed>: glue_port.paf_to_pose (the oracle's NMS, then the reference's pafprocess)
+        as humans rows [k, 1 + 18 * 3] in float64, exact."""
+    from oracle import glue_port
+    pafprocess_oracle.build(ref=True)
+    ref = pafprocess_oracle.load_ref()
+    digests, counts, scores, cids, parts = [], [], [], [], []
+    for t in range(FUZZ_SCENARIOS):
+        h, w, jl, paf = synth.fuzz_scenario(t)
+        digests.append(digest(jl, paf))
+        if len(jl) == 0:
+            counts.append(-1)
+            continue
+        paf_up = np.ascontiguousarray(np.repeat(np.repeat(paf, 8, axis=0), 8, axis=1))
+        ref.process_paf(jl[None], np.zeros((h * 8, w * 8, 19), np.float32), paf_up)
+        counts.append(ref.get_num_humans())
+        for hid in range(ref.get_num_humans()):
+            scores.append(ref.get_score(hid))
+            c = [int(ref.get_part_cid(hid, p)) for p in range(18)]
+            cids.append(c)
+            parts.append([(ref.get_part_x(k), ref.get_part_y(k), ref.get_part_score(k)) if k >= 0 else (-1, -1, -1)
+                          for k in c])
+    out = dict(fuzz_digest=np.array(digests), fuzz_humans=np.array(counts, np.int32),
+               fuzz_score=np.array(scores, np.float32), fuzz_cid=np.array(cids, np.int32).reshape(-1, 18),
+               fuzz_part=np.array(parts, np.float64).reshape(-1, 18, 3))
+
+    def rows(humans):
+        r = np.full((len(humans), 1 + 18 * 3), -1.0, np.float64)
+        for i, (score, body) in enumerate(humans):
+            r[i, 0] = score
+            for p, v in body.items():
+                r[i, 1 + 3 * p: 4 + 3 * p] = v
+        return r
+    for name, (heat, paf) in post_cases():
+        out["post_" + name] = rows(glue_port.paf_to_pose(heat, paf, ref)[1])
+    for persons, seed in TIES_CASES:
+        heat, paf, _ = synth.stick_figures(persons, seed)
+        out["ties_%d_%d" % (persons, seed)] = rows(glue_port.paf_to_pose(heat, paf, ref)[1])
+    np.savez_compressed(os.path.join(OUT, "pafprocess_ref.npz"), **out)
+    print("pafprocess: %d fuzz scenarios, %d humans" % (FUZZ_SCENARIOS, len(scores)))
+
+
+def make_scripts():
+    """The reference's demo/picture_demo.py and evaluate/evaluation.py executed unmodified from this repository's root
+    up to their first .cuda(), as tests/test_reference_scripts.py does: the record of each run.  Runs in a process of
+    its own, with this repository's lib.* / evaluate.* (import_reference() puts the reference's in their place)."""
+    import json
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_reference_scripts
+    sd = net_port.he_state_dict(1234)
+    ckpt = {"state_dict": {"model." + k: v for k, v in sd.items()}}
+    out = {}
+    for rel, ckpt_of in (("demo/picture_demo.py", sd), ("evaluate/evaluation.py", ckpt)):
+        out[rel] = test_reference_scripts.run_reference_script(os.path.join(REF, rel), lambda *a, **k: ckpt_of)[1]
+        print(rel, "reaches .cuda() on", out[rel]["cuda_on"], "after", len(out[rel]["imports"]), "imports")
+    with open(os.path.join(OUT, "reference_scripts.json"), "w") as f:
+        json.dump(out, f, indent=1)
+        f.write("\n")
+
+
 def main():
     import torch
+    if ARGS == ["scripts"]:
+        make_scripts()
+        return
+    if not ARGS or "scripts" in ARGS:
+        import subprocess
+        subprocess.run([sys.executable, os.path.abspath(__file__), "scripts"], check=True)
+    if not ARGS or "paf" in ARGS:
+        make_pafprocess()           # needs only the compiled pafprocess.cpp
+    if ARGS and set(ARGS) <= {"paf", "scripts"}:
+        return
     get_model, ref_p2p, ref_eval, cfg = import_reference()
     if not ARGS or "pre" in ARGS:
         make_preprocess()
@@ -155,7 +239,7 @@ def main():
         make_crop()
     if not ARGS or "eval" in ARGS:
         make_eval(ref_eval)
-    if ARGS and set(ARGS) <= {"crop", "eval", "pre"}:
+    if ARGS and set(ARGS) <= {"crop", "eval", "pre", "paf", "scripts"}:
         return
     torch.manual_seed(0)
 
@@ -190,11 +274,7 @@ def main():
     np.savez_compressed(os.path.join(OUT, "flip_merge.npz"), avg_paf=ap, avg_heat=ah)
 
     # ---------------- post-processing (NMS + paf_to_pose_cpp with the compiled pafprocess.cpp) ----------------
-    cases = [("p1", synth.stick_figures(1, 1)[:2]), ("p3", synth.stick_figures(3, 3)[:2]),
-             ("p8", synth.stick_figures(8, 8)[:2]), ("p30", synth.stick_figures(30, 30)[:2]),
-             ("noise0", synth.noise_maps(0)), ("empty", (np.zeros((46, 46, 19), np.float32), np.zeros((46, 46, 38), np.float32))),
-             ("p5_40x52", synth.stick_figures(5, 55, h=40, w=52)[:2])]
-    for name, (heat, paf) in cases:
+    for name, (heat, paf) in post_cases():
         per_joint = ref_p2p.NMS(heat, upsampFactor=cfg.MODEL.DOWNSAMPLE, config=cfg)
         jl = np.array([tuple(p) + (j,) for j, peaks in enumerate(per_joint) for p in peaks]).astype(np.float32).reshape(-1, 5)
         humans = ref_p2p.paf_to_pose_cpp(heat, paf, cfg)

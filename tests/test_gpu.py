@@ -442,7 +442,7 @@ def test_data_parallel_over_every_visible_gpu(built, he_sd):
     print("DataParallel over %d GPU(s): identical to the single-device forward" % ngpu)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_rank_sharded_batch_equals_single_gpu(built, he_sd, tmp_path):
     """SURVEY.md 4 / 8(e): a batch sharded over two ranks (one process per GPU, NCCL weight broadcast, shard_range)
     gives, frame by frame, bit-identical persons to the same batch on one GPU."""

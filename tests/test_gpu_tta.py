@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, assert_humans_equal, golden, pkg_module
+from conftest import ROOT, RecordedPafprocess, assert_humans_equal, golden, pkg_module
 from oracle import glue_port, pafprocess_oracle, synth
 
 pytestmark = pytest.mark.gpu
@@ -90,25 +90,19 @@ def test_fused_flip_inference_matches_reference_shaped_composition(built, he_sd)
 def test_pafprocess_kernels_fuzz_against_the_compiled_reference(built):
     """The limbs / assembly kernels (through the legacy lib.pafprocess surface: joint list + x8 maps, exactly what the
     SWIG module gets) on 80 random inputs the fixtures do not reach - duplicated peaks on one pixel, exact score ties,
-    cross links between persons, masked fields - against the reference's own pafprocess.cpp (oracle/_ref; the C port
-    when it is absent).  Same scenario generator as the host-side fuzz in tests/test_host.py."""
+    cross links between persons, masked fields - against what the reference's own pafprocess.cpp returned on them
+    (golden).  Same scenarios as the host-side fuzz in tests/test_host.py."""
     from lib.pafprocess import pafprocess
-    ref = pafprocess_oracle.load_ref() if pafprocess_oracle.have_ref() else pafprocess_oracle.load_port()
+    ref = RecordedPafprocess()
     humans = 0
     for t in range(80):
-        rs = np.random.RandomState(1000 + t)
-        h, w = int(rs.choice([12, 23, 46])), int(rs.choice([23, 46, 53]))
-        if t % 2:
-            h = max(h, 23)
-            jl, paf = synth.fuzz_persons(rs, h, w)
-        else:
-            jl, paf = synth.fuzz_field(rs, h, w, ("uniform", "cluster", "ties")[(t // 2) % 3])
+        h, w, jl, paf = synth.fuzz_scenario(t)
         if len(jl) == 0:
             continue
         paf_up = np.ascontiguousarray(np.repeat(np.repeat(paf, 8, 0), 8, 1))
         heat_up = np.zeros((h * 8, w * 8, 19), np.float32)
         assert pafprocess.process_paf(jl[None], heat_up, paf_up) == 0
-        ref.process_paf(jl[None], heat_up, paf_up)
+        ref.select(t, jl, paf)
         assert pafprocess.get_num_humans() == ref.get_num_humans(), "scenario seed %d" % (1000 + t)
         for hid in range(ref.get_num_humans()):
             assert pafprocess.get_score(hid) == ref.get_score(hid), "scenario seed %d" % (1000 + t)

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import POST_CASES, ROOT, assert_humans_equal, golden, pkg_module
+from conftest import POST_CASES, ROOT, RecordedPafprocess, assert_humans_equal, golden, pkg_module
 from oracle import glue_port, net_port, nms_port, pafprocess_oracle, synth
 
 
@@ -386,19 +386,18 @@ def test_device_cores_on_host_match_oracle(name, built):
 
 def test_device_cores_on_host_fuzz_against_the_compiled_reference(built):
     """300 random pafprocess inputs (peak sets with clusters / duplicated pixels, direction fields with exact ties, person
-    shapes with cross links) through csrc/post_core.h on the host and through the reference's own pafprocess.cpp
-    (oracle/_ref; the C port when the reference sources are absent): identical persons, scores and part assignments."""
+    shapes with cross links) through csrc/post_core.h on the host, against what the reference's own pafprocess.cpp
+    returned on them (golden): identical persons, scores and part assignments."""
     lib = ctypes.CDLL(os.path.join(ROOT, "build", "libpostcore_host.so"))
     FP = ctypes.POINTER(ctypes.c_float)
     lib.core_process.argtypes = [ctypes.c_int, FP, ctypes.c_int, FP, ctypes.c_long, ctypes.c_long, ctypes.c_long,
                                  ctypes.c_int, ctypes.c_int]
     lib.core_result.restype = FP
-    ref = pafprocess_oracle.load_ref() if pafprocess_oracle.have_ref() else pafprocess_oracle.load_port()
+    ref = RecordedPafprocess()
     to_dicts = pkg_module("engine").humans_to_dicts
 
-    def ref_humans(jl, paf, h, w):
-        paf_up = np.ascontiguousarray(np.repeat(np.repeat(paf, 8, axis=0), 8, axis=1))
-        ref.process_paf(jl[None], np.zeros((h * 8, w * 8, 19), np.float32), paf_up)
+    def ref_humans(t, jl, paf, h, w):
+        ref.select(t, jl, paf)
         out = []
         for hid in range(ref.get_num_humans()):
             parts = {}
@@ -412,16 +411,10 @@ def test_device_cores_on_host_fuzz_against_the_compiled_reference(built):
         return out
     humans = 0
     for t in range(300):
-        rs = np.random.RandomState(1000 + t)
-        h, w = int(rs.choice([12, 23, 46])), int(rs.choice([23, 46, 53]))
-        if t % 2:
-            h = max(h, 23)
-            jl, paf = synth.fuzz_persons(rs, h, w)
-        else:
-            jl, paf = synth.fuzz_field(rs, h, w, ("uniform", "cluster", "ties")[(t // 2) % 3])
+        h, w, jl, paf = synth.fuzz_scenario(t)
         if len(jl) == 0:
             continue
-        want = ref_humans(jl, paf, h, w)
+        want = ref_humans(t, jl, paf, h, w)
         nh = lib.core_process(len(jl), jl.ctypes.data_as(FP), h * 8, paf.ctypes.data_as(FP), 1, w * 38, 38, 3, 0)
         rows = (np.ctypeslib.as_array(lib.core_result(), shape=(nh * 73,)).reshape(nh, 73).copy() if nh else
                 np.zeros((0, 73), np.float32))

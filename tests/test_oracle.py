@@ -1,5 +1,5 @@
 """CPU: pins the oracle (CPU restatements under oracle/) against golden vectors produced by the unmodified
-reference (tests/golden/make_golden.py) and against the compiled reference pafprocess.cpp."""
+reference and its compiled pafprocess.cpp (tests/golden/make_golden.py)."""
 import hashlib
 import itertools
 
@@ -123,20 +123,18 @@ def test_pafprocess_port_matches_reference(name, built):
     port = pafprocess_oracle.load_port()
     _, humans = glue_port.paf_to_pose(heat, paf, port)
     assert_humans_equal(humans, humans_rows_to_dicts(g["humans"]), score_tol=1e-6)
-    if pafprocess_oracle.have_ref():      # the reference's own translation unit, same peaks -> bit-identical
-        _, href = glue_port.paf_to_pose(heat, paf, pafprocess_oracle.load_ref())
-        assert humans == href
+    # the reference's own translation unit on the same peaks (golden) -> bit-identical
+    assert humans == humans_rows_to_dicts(golden("pafprocess_ref")["post_" + name])
 
 
 def test_pafprocess_port_ties_and_scale(built):
-    """Large crowded scenes produce exactly-equal candidate scores; std::sort's order is reproduced."""
-    if not pafprocess_oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    port, ref = pafprocess_oracle.load_port(), pafprocess_oracle.load_ref()
+    """Large crowded scenes produce exactly-equal candidate scores; std::sort's order is reproduced (golden: the
+    reference's own pafprocess.cpp on the same scenes)."""
+    port, ref = pafprocess_oracle.load_port(), golden("pafprocess_ref")
     for persons, seed in [(30, 31), (50, 5), (80, 7)]:
         heat, paf, _ = synth.stick_figures(persons, seed)
         a = glue_port.paf_to_pose(heat, paf, port)[1]
-        b = glue_port.paf_to_pose(heat, paf, ref)[1]
+        b = humans_rows_to_dicts(ref["ties_%d_%d" % (persons, seed)])
         assert a == b and len(a) > persons // 2
 
 
