@@ -71,6 +71,17 @@ int b200pose_net_forward_u8(b200pose_net* net, const unsigned char* images, int 
 #define B200POSE_PRE_INCEPTION 3   /* BGR -> RGB, x/128 - 1                         */
 #define B200POSE_PRE_SSD 4         /* x - (123, 117, 104) on (B, G, R)              */
 int b200pose_net_set_preprocess(b200pose_net* net, int preprocess);
+/* Ragged batch: n already-cropped uint8 BGR frames of DIFFERENT sizes in one [n,H,W,3] canvas, frame i valid in
+ * [0,ext_h[i]) x [0,ext_w[i]) of its slot (top-left corner).  ext_h / ext_w: host arrays of n extents, each a multiple
+ * of 8 in [8, H] / [8, W] (H, W: multiples of 8, normally the largest extents).  Canvas bytes outside an extent are not
+ * read.  outputs[12] as for b200pose_net_forward_u8, canvas-shaped ([n,C,H/8,W/8]); inside (ext_h[i]/8, ext_w[i]/8)
+ * every value is bit-identical to b200pose_net_forward_u8 of frame i alone (same mode), outside it is exactly +0.
+ * Every layer still computes the whole canvas: the cost is that of n frames of H x W.  Ragged calls always launch
+ * directly (no CUDA graph).  Errors (no fault): null extent arrays, an extent that is not a multiple of 8 or exceeds
+ * the canvas, n outside [1, 4096]. */
+int b200pose_net_forward_u8_ragged(b200pose_net* net, const unsigned char* canvas, int input_on_device, int n, int H,
+                                   int W, const int* ext_h, const int* ext_w, int mode, float* const* outputs,
+                                   int outputs_on_device, void* cuda_stream);
 /* Measurement hook: re-runs the launch list of the last bf16 forward (conv1_1 + 51 tensor-core launches) with a CUDA
  * event pair around every launch; fills per-launch milliseconds and ALGORITHMIC FLOPs (2 x MACs of the unpadded
  * convolution).  Returns the number of launches, < 0 on error. */
@@ -177,6 +188,21 @@ int b200pose_net_crop_with_factor(b200pose_net* net, const unsigned char* images
 int b200pose_infer_raw_u8(b200pose_net* net, b200pose_post* post, const unsigned char* images, int input_on_device, int n,
                           int src_h, int src_w, int dest_size, int factor, int mode, float thresh, int flip,
                           void* cuda_stream);
+/* Ragged batch of raw frames of different sizes: frame i is [src_h[i],src_w[i],3] uint8 BGR, the frames packed back to
+ * back in `frames` (frame i starts at byte sum_{j<i} 3 src_h[j] src_w[j]; host or device).  Each frame gets its own
+ * crop_with_factor(dest_size, factor) as in b200pose_infer_raw_u8, all n then run through the network and the fused
+ * post-processing as ONE batch on a canvas of the largest padded height x the largest padded width.  Person rows of
+ * frame i equal those of b200pose_infer_raw_u8 on frame i alone, in pixels of frame i's own padded frame.  Results are
+ * fetched like b200pose_infer's (tickets, two runs in flight); a host input stays alive until then.  No flip.
+ * Errors (no fault): null pointers, n < 1 or n > the post's batch_cap, a frame size crop_with_factor rejects. */
+int b200pose_infer_raw_u8_ragged(b200pose_net* net, b200pose_post* post, const unsigned char* frames,
+                                 int input_on_device, int n, const int* src_h, const int* src_w, int dest_size,
+                                 int factor, int mode, float thresh, void* cuda_stream);
+/* Host only: the layout b200pose_infer_raw_u8_ragged gives n raw frames - per frame its byte offset in the packed input
+ * (src_off[n]) and its padded size (pad_h[n], pad_w[n], as b200pose_crop_geometry reports for it alone), and the canvas
+ * (largest pad_h x largest pad_w).  Errors: null pointers, n < 1, a frame size crop_with_factor rejects. */
+int b200pose_ragged_layout(int n, const int* src_h, const int* src_w, int dest_size, int factor, long* src_off,
+                           int* pad_h, int* pad_w, int* canvas_h, int* canvas_w);
 
 /* Multi-scale (+ flip) test-time averaging, BASELINE.json configs[4].  The reference at this commit has no multi-scale
  * loop (get_outputs is single-scale, evaluate/coco_eval.py:87-91); the protocol is composed from its own functions:

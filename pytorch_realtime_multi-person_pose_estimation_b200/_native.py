@@ -41,6 +41,9 @@ def lib():
         "b200pose_net_forward": ([vp, vp, ci, ci, ci, ci, ci, ctypes.POINTER(vp), ci, vp], ci),
         "b200pose_net_forward_u8": ([vp, vp, ci, ci, ci, ci, ci, ctypes.POINTER(vp), ci, vp], ci),
         "b200pose_net_set_preprocess": ([vp, ci], ci),
+        "b200pose_net_forward_u8_ragged": ([vp, vp, ci, ci, ci, ci, vp, vp, ci, ctypes.POINTER(vp), ci, vp], ci),
+        "b200pose_infer_raw_u8_ragged": ([vp, vp, vp, ci, ci, vp, vp, ci, ci, ci, cf, vp], ci),
+        "b200pose_ragged_layout": ([ci, vp, vp, ci, ci, vp, vp, vp, ctypes.POINTER(ci), ctypes.POINTER(ci)], ci),
         "b200pose_net_profile": ([vp, vp, vp, ci, vp], ci),
         "b200pose_net_last_maps": ([vp, ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(ci), ctypes.POINTER(ci),
                                     ctypes.POINTER(ci)], ci),
@@ -89,7 +92,8 @@ EXPORTED = ["b200pose_last_error", "b200pose_version", "b200pose_launch_count", 
             "b200pose_post_run", "b200pose_post_sync", "b200pose_post_last_ticket", "b200pose_post_select", "b200pose_post_debug", "b200pose_post_debug_sort", "b200pose_post_status_accum", "b200pose_post_num_humans", "b200pose_post_status",
             "b200pose_post_get_humans", "b200pose_post_get_peaks", "b200pose_infer", "b200pose_infer_u8", "b200pose_flip_merge", "b200pose_infer_flip",
             "b200pose_infer_u8_flip", "b200pose_crop_geometry", "b200pose_net_crop_with_factor",
-            "b200pose_infer_raw_u8", "b200pose_infer_raw_u8_multiscale", "process_paf", "get_num_humans",
+            "b200pose_infer_raw_u8", "b200pose_infer_raw_u8_multiscale", "b200pose_net_forward_u8_ragged",
+            "b200pose_infer_raw_u8_ragged", "b200pose_ragged_layout", "process_paf", "get_num_humans",
             "get_part_cid", "get_score", "get_part_x", "get_part_y", "get_part_score"]
 
 
@@ -107,6 +111,20 @@ def crop_geometry(src_h, src_w, dest_size=368, factor=8):
     check(lib().b200pose_crop_geometry(int(src_h), int(src_w), int(dest_size), int(factor), ctypes.byref(sc),
                                        *[ctypes.byref(x) for x in v]), "b200pose_crop_geometry")
     return sc.value, (v[0].value, v[1].value), (v[2].value, v[3].value)
+
+
+def ragged_layout(src_sizes, dest_size=368, factor=8):
+    """Layout of a ragged batch of raw frames [(src_h, src_w), ...] packed back to back, as b200pose_infer_raw_u8_ragged
+    computes it: (byte offset of each frame, [(pad_h, pad_w)] per frame, (canvas_h, canvas_w)).  Host arithmetic only."""
+    n = len(src_sizes)
+    sh = (ctypes.c_int * max(n, 1))(*[int(h) for h, _ in src_sizes])
+    sw = (ctypes.c_int * max(n, 1))(*[int(w) for _, w in src_sizes])
+    off = (ctypes.c_long * max(n, 1))()
+    ph, pw = (ctypes.c_int * max(n, 1))(), (ctypes.c_int * max(n, 1))()
+    ch, cw = ctypes.c_int(), ctypes.c_int()
+    check(lib().b200pose_ragged_layout(n, sh, sw, int(dest_size), int(factor), off, ph, pw, ctypes.byref(ch),
+                                       ctypes.byref(cw)), "b200pose_ragged_layout")
+    return list(off[:n]), list(zip(ph[:n], pw[:n])), (ch.value, cw.value)
 
 
 def launch_count():

@@ -47,6 +47,7 @@ const ConvSpec kTrunk[12] = {{3, 64, 3},    {64, 64, 3},   {64, 128, 3},  {128, 
                              {256, 256, 3}, {256, 256, 3}, {256, 512, 3}, {512, 512, 3}, {512, 256, 3}, {256, 128, 3}};
 const bool kPoolAfter[12] = {false, true, false, true, false, false, false, true, false, false, false, false};
 constexpr int kPaf = 38, kHeat = 19, kFeat = 128, kCat = kPaf + kHeat + kFeat;
+constexpr int kRaggedCap = 4096;       // images per ragged call (size of the net's fixed extent array)
 
 int stage_num_layers(int stage) { return stage == 1 ? 5 : 7; }
 ConvSpec stage_layer(int stage, int branch, int li) {
@@ -145,6 +146,7 @@ struct b200pose_net {
     // into have not been reallocated.  B200POSE_PLAN_CACHE=0 (read when the net is created) turns it off.
     struct PlanEntry {
         int n, H, W, mode;
+        bool ragged;
         bool split;
         std::vector<ConvTcArgs> plan;
         std::vector<double> flops;
@@ -173,6 +175,7 @@ struct b200pose_net {
     std::map<GraphKey, cudaGraphExec_t> graphs;
     std::set<GraphKey> graph_seen;    // a key is captured at its SECOND use: callers that pass a fresh pointer every time never pay a capture
     int kn = 0, kH = 0, kW = 0, kmode = -1;      // key of the plan currently held in `plan`
+    bool kragged = false, pragged = false;       // ... and whether it (resp. the last bf16 forward's plan) is a ragged plan
     std::vector<PlanEntry> plan_cache;
     DevBuf<__nv_bfloat16> t1, t2, t3, t4, t5a, t5b, t6, t7, t8, t9, cat, bra, brb, br512;
     // residual ("lo") planes of the same buffers, split-precision mode only
@@ -187,6 +190,10 @@ struct b200pose_net {
     DevBuf<unsigned char> in_stage_u8;
     int preprocess = 1;                // normalisation fused into the uint8 entry points (preprocess_core.h; 1 = rtpose)
     DevBuf<unsigned char> raw_stage;   // raw (un-resized) frames of b200pose_*crop* / b200pose_infer_raw_u8
+    // Ragged batches: full-resolution (h, w) of every image of the call, uploaded on the caller's stream before its first
+    // launch.  Allocated once at kRaggedCap entries: the ragged plans (their ConvTcArgs::ext) point into it.
+    DevBuf<int2> ext;
+    DevBuf<RaggedCrop> rcrop;          // per-frame crop geometry of b200pose_infer_raw_u8_ragged
 };
 
 struct b200pose_post {
@@ -216,6 +223,7 @@ struct b200pose_post {
     // profiles/r02_variants.txt).  B200POSE_POST_OVERLAP=0 keeps everything on the caller's stream.
     bool overlap = true;
     DevBuf<float> ov_maps[2];                       // [heat | paf] copies, slot = run parity
+    DevBuf<int2> dims[2];                           // ragged runs: low-res (h, w) per image, slot = run parity
     cudaEvent_t ev_maps = nullptr, ev_ld[2] = {nullptr, nullptr};   // maps copied (st) / limbs done with a slot (s2)
     bool have_ld[2] = {false, false};
 };
@@ -315,7 +323,7 @@ int add_plan(b200pose_net* net, const TcLayer& L, int n, int H, int W, const __n
     return 0;
 }
 
-int build_plan_bf16(b200pose_net* net, int n, int H, int W, bool split, cudaStream_t st) {
+int build_plan_bf16(b200pose_net* net, int n, int H, int W, bool split, bool ragged, cudaStream_t st) {
     const size_t px1 = (size_t)n * H * W, px2 = px1 / 4, px4 = px1 / 16, px8 = px1 / 64;
     const int h = H / 8, w = W / 8;
     CU(net->t1.ensure(px1 * 64)); CU(net->t2.ensure(px2 * 64)); CU(net->t3.ensure(px2 * 128));
@@ -377,6 +385,12 @@ int build_plan_bf16(b200pose_net* net, int n, int H, int W, bool split, cudaStre
              net->out_f32[2 * (s - 1)].p, net->out_f32[2 * (s - 1) + 1].p, kPaf, kHeat);
     }
 #undef PLAN
+    if (ragged)      // every layer masks by the images' extents at its input resolution H >> ext_shift
+        for (ConvTcArgs& a : net->plan) {
+            a.ext = net->ext.p;
+            a.ext_shift = 0;
+            while ((H >> a.ext_shift) > a.H) ++a.ext_shift;
+        }
     return 0;
 }
 
@@ -390,17 +404,18 @@ std::vector<const void*> plan_buffers(const b200pose_net* net) {
 }
 
 // plan cache (experiment): returns true when a valid plan for the key was swapped into net->plan
-bool plan_cache_swap(b200pose_net* net, int n, int H, int W, int want) {
+bool plan_cache_swap(b200pose_net* net, int n, int H, int W, int want, bool ragged) {
     if (net->kmode >= 0 && !net->plan.empty()) {      // stash the plan we hold
         b200pose_net::PlanEntry* slot = nullptr;
         for (auto& e : net->plan_cache)
-            if (e.n == net->kn && e.H == net->kH && e.W == net->kW && e.mode == net->kmode) slot = &e;
+            if (e.n == net->kn && e.H == net->kH && e.W == net->kW && e.mode == net->kmode && e.ragged == net->kragged) slot = &e;
         if (!slot) {
             if (net->plan_cache.size() >= 32) net->plan_cache.erase(net->plan_cache.begin());
             net->plan_cache.emplace_back();
             slot = &net->plan_cache.back();
         }
-        slot->n = net->kn; slot->H = net->kH; slot->W = net->kW; slot->mode = net->kmode; slot->split = net->plan_split;
+        slot->n = net->kn; slot->H = net->kH; slot->W = net->kW; slot->mode = net->kmode; slot->ragged = net->kragged;
+        slot->split = net->plan_split;
         slot->plan.swap(net->plan);
         slot->flops.swap(net->plan_flops);
         slot->buffers = plan_buffers(net);
@@ -408,11 +423,12 @@ bool plan_cache_swap(b200pose_net* net, int n, int H, int W, int want) {
         net->kmode = -1;
     }
     for (auto& e : net->plan_cache)
-        if (e.n == n && e.H == H && e.W == W && e.mode == want && !e.plan.empty() && e.buffers == plan_buffers(net)) {
+        if (e.n == n && e.H == H && e.W == W && e.mode == want && e.ragged == ragged && !e.plan.empty() &&
+            e.buffers == plan_buffers(net)) {
             net->plan.swap(e.plan);
             net->plan_flops.swap(e.flops);
             net->plan_split = e.split;
-            net->kn = n; net->kH = H; net->kW = W; net->kmode = want;
+            net->kn = n; net->kH = H; net->kW = W; net->kmode = want; net->kragged = ragged;
             return true;
         }
     return false;
@@ -424,24 +440,32 @@ void drop_graphs(b200pose_net* net) {
     net->graph_seen.clear();
 }
 
-int launch_forward_bf16(b200pose_net* net, const void* d_in, int in_u8, int n, int H, int W, cudaStream_t st, bool split) {
-    CU(conv_first_launch(d_in, in_u8, net->d_w[0], net->d_b[0], net->t1.p, split ? net->l1.p : nullptr, n, H, W, st));
+int launch_forward_bf16(b200pose_net* net, const void* d_in, int in_u8, int n, int H, int W, cudaStream_t st, bool split,
+                        const int2* ext = nullptr) {
+    CU(conv_first_launch(d_in, in_u8, net->d_w[0], net->d_b[0], net->t1.p, split ? net->l1.p : nullptr, n, H, W, st, ext));
     for (const ConvTcArgs& a : net->plan) CU(conv_tc_launch(a, net->num_sms, st));
     return 0;
 }
 
-int forward_bf16(b200pose_net* net, const void* d_in, int in_u8, int n, int H, int W, cudaStream_t st, bool split) {
+// ragged: the images' extents are in net->ext (the plan masks by them); such calls always launch directly, never as a graph
+int forward_bf16(b200pose_net* net, const void* d_in, int in_u8, int n, int H, int W, cudaStream_t st, bool split,
+                 bool ragged = false) {
     const int want = split ? B200POSE_MODE_BF16X3 : B200POSE_MODE_BF16;
-    if (net->pn != n || net->pH != H || net->pW != W || net->pmode != want) {
-        if (!(net->plan_cache_on && plan_cache_swap(net, n, H, W, want))) {
+    if (net->pn != n || net->pH != H || net->pW != W || net->pmode != want || net->pragged != ragged) {
+        if (!(net->plan_cache_on && plan_cache_swap(net, n, H, W, want, ragged))) {
             CU(cudaStreamSynchronize(st));
             drop_graphs(net);                   // the buffers the captured tensor maps point into may move
-            if (build_plan_bf16(net, n, H, W, split, st)) return 1;
-            net->kn = n; net->kH = H; net->kW = W; net->kmode = want;
+            if (build_plan_bf16(net, n, H, W, split, ragged, st)) return 1;
+            net->kn = n; net->kH = H; net->kW = W; net->kmode = want; net->kragged = ragged;
         }
-        net->pn = n; net->pH = H; net->pW = W; net->pmode = want;
+        net->pn = n; net->pH = H; net->pW = W; net->pmode = want; net->pragged = ragged;
     }
     const long launches = 1 + (long)net->plan.size();
+    if (ragged) {
+        if (launch_forward_bf16(net, d_in, in_u8, n, H, W, st, split, net->ext.p)) return 1;
+        g_launches += launches;
+        return 0;
+    }
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     if (net->use_graph && small_plan(net, n, H, W) && st != nullptr && cudaStreamIsCapturing(st, &cap) == cudaSuccess &&
         cap == cudaStreamCaptureStatusNone) {
@@ -482,7 +506,7 @@ int forward_bf16(b200pose_net* net, const void* d_in, int in_u8, int n, int H, i
     return 0;
 }
 
-int forward_fp32(b200pose_net* net, const float* d_in, int n, int H, int W, cudaStream_t st) {
+int forward_fp32(b200pose_net* net, const float* d_in, int n, int H, int W, cudaStream_t st, const int2* ext = nullptr) {
     const size_t px1 = (size_t)n * H * W;
     const int h = H / 8, w = W / 8;
     const size_t px8 = (size_t)n * h * w;
@@ -504,6 +528,8 @@ int forward_fp32(b200pose_net* net, const float* d_in, int n, int H, int W, cuda
         a.in = in; a.in_cstride = in_cs; a.in_ch_off = in_off; a.w = net->d_w[ci]; a.bias = net->d_b[ci];
         a.out = out; a.out_cstride = out_cs; a.out_ch_off = out_off; a.out_nchw = nchw;
         a.n_img = n; a.H = hh; a.W = ww; a.cin = s.cin; a.cout = s.cout; a.ks = s.ks; a.relu = relu;
+        a.ext = ext; a.ext_shift = 0;
+        while ((H >> a.ext_shift) > hh) ++a.ext_shift;
         CU(conv_f32_launch(a, st));
         ++g_launches;
         return 0;
@@ -606,6 +632,8 @@ void b200pose_net_destroy(b200pose_net* net) {
     DevBuf<float>* fb[] = {&net->in_stage, &net->f_a, &net->f_b, &net->f_cat, &net->f_x, &net->f_y, &net->f_in, &net->f_u8};
     net->in_stage_u8.release();
     net->raw_stage.release();
+    net->ext.release();
+    net->rcrop.release();
     for (auto* b : fb) b->release();
     for (auto& b : net->out_f32) b.release();
     delete net;
@@ -668,11 +696,35 @@ int b200pose_net_finalize(b200pose_net* net) {
     return 0;
 }
 
+// Extents of a ragged call: n host (h, w) pairs, each a multiple of 8 in [8, H] x [8, W].
+static int ragged_check(int n, int H, int W, const int* ext_h, const int* ext_w) {
+    if (!ext_h || !ext_w) return fail("ragged: null extent array");
+    if (n < 1 || n > kRaggedCap) return fail("ragged: batch %d outside [1, %d]", n, kRaggedCap);
+    for (int i = 0; i < n; ++i)
+        if (ext_h[i] < 8 || ext_w[i] < 8 || ext_h[i] % 8 || ext_w[i] % 8 || ext_h[i] > H || ext_w[i] > W)
+            return fail("ragged: extent %d is %d x %d; extents must be multiples of 8 within the %d x %d canvas", i, ext_h[i],
+                        ext_w[i], H, W);
+    return 0;
+}
+
+// ext_h / ext_w (host, may be null): a ragged batch, see b200pose_net_forward_u8_ragged (uint8 input only).
 static int net_forward_impl(b200pose_net* net, const void* input, int in_u8, int input_on_device, int n, int H, int W,
-                            int mode, float* const* outputs, int outputs_on_device, cudaStream_t st, bool sync_host) {
+                            int mode, float* const* outputs, int outputs_on_device, cudaStream_t st, bool sync_host,
+                            const int* ext_h = nullptr, const int* ext_w = nullptr) {
     if (!net || !net->finalized) return fail("net not finalized");
     if (n < 1 || H < 8 || W < 8 || (H % 8) || (W % 8)) return fail("input must be [n,3,H,W] with H, W multiples of 8");
+    const bool ragged = ext_h != nullptr || ext_w != nullptr;
+    if (ragged && !in_u8) return fail("ragged batches take uint8 frames");
+    if (ragged && ragged_check(n, H, W, ext_h, ext_w)) return 1;
     CU(cudaSetDevice(net->device));
+    if (ragged) {
+        // stream-ordered after the previous call's launches, which may still read the extent array
+        CU(net->ext.ensure(kRaggedCap));
+        std::vector<int2> e(n);
+        for (int i = 0; i < n; ++i) e[i] = make_int2(ext_h[i], ext_w[i]);
+        CU(cudaMemcpyAsync(net->ext.p, e.data(), n * sizeof(int2), cudaMemcpyHostToDevice, st));
+    }
+    const int2* d_ext = ragged ? net->ext.p : nullptr;
     const void* d_in = input;
     const size_t elems = (size_t)n * 3 * H * W;
     if (!input_on_device) {
@@ -690,11 +742,12 @@ static int net_forward_impl(b200pose_net* net, const void* input, int in_u8, int
     if (mode == B200POSE_MODE_FP32) {
         if (in_u8) {   // parity mode: materialise rtpose_preprocess, then the fp32 path
             CU(net->f_u8.ensure(elems));
-            CU(u8hwc_to_f32nchw_launch(static_cast<const unsigned char*>(d_in), net->f_u8.p, n, H, W, net->preprocess, st));
+            CU(u8hwc_to_f32nchw_launch(static_cast<const unsigned char*>(d_in), net->f_u8.p, n, H, W, net->preprocess, st,
+                                       d_ext));
             ++g_launches;
-            rc = forward_fp32(net, net->f_u8.p, n, H, W, st);
+            rc = forward_fp32(net, net->f_u8.p, n, H, W, st, d_ext);
         } else rc = forward_fp32(net, static_cast<const float*>(d_in), n, H, W, st);
-    } else rc = forward_bf16(net, d_in, in_u8 ? net->preprocess : 0, n, H, W, st, mode == B200POSE_MODE_BF16X3);
+    } else rc = forward_bf16(net, d_in, in_u8 ? net->preprocess : 0, n, H, W, st, mode == B200POSE_MODE_BF16X3, ragged);
     if (rc) return rc;
     net->last_in = d_in;
     net->last_in_u8 = (mode == B200POSE_MODE_FP32) ? 0 : (in_u8 ? net->preprocess : 0);
@@ -722,6 +775,14 @@ int b200pose_net_forward_u8(b200pose_net* net, const unsigned char* images, int 
                             reinterpret_cast<cudaStream_t>(cuda_stream), true);
 }
 
+int b200pose_net_forward_u8_ragged(b200pose_net* net, const unsigned char* canvas, int input_on_device, int n, int H,
+                                   int W, const int* ext_h, const int* ext_w, int mode, float* const* outputs,
+                                   int outputs_on_device, void* cuda_stream) {
+    if (!ext_h || !ext_w) return fail("ragged: null extent array");
+    return net_forward_impl(net, canvas, 1, input_on_device, n, H, W, mode, outputs, outputs_on_device,
+                            reinterpret_cast<cudaStream_t>(cuda_stream), true, ext_h, ext_w);
+}
+
 int b200pose_net_set_preprocess(b200pose_net* net, int preprocess) {
     if (!net) return fail("null net");
     if (preprocess < 1 || preprocess > 4) return fail("preprocess must be 1 (rtpose), 2 (vgg), 3 (inception) or 4 (ssd)");
@@ -743,7 +804,7 @@ int b200pose_net_profile(b200pose_net* net, float* ms, double* flops, int cap, v
     if (!d_in) { if (tmp.ensure((size_t)n * 3 * H * W) != cudaSuccess) return -1; cudaMemsetAsync(tmp.p, 0, (size_t)n * 3 * H * W * 4, st); d_in = tmp.p; net->last_in_u8 = 0; }
     cudaEventRecord(ev[0], st);
     conv_first_launch(d_in, net->last_in_u8, net->d_w[0], net->d_b[0], net->t1.p, net->plan_split ? net->l1.p : nullptr, n, H, W,
-                      st);
+                      st, net->pragged ? net->ext.p : nullptr);
     cudaEventRecord(ev[1], st);
     for (size_t i = 0; i < net->plan.size(); ++i) {
         conv_tc_launch(net->plan[i], net->num_sms, st);
@@ -807,6 +868,7 @@ void b200pose_post_destroy(b200pose_post* p) {
     p->d_heat.release(); p->d_paf.release();
     p->tta_in.release(); p->tta_out.release();
     p->ov_maps[0].release(); p->ov_maps[1].release();
+    p->dims[0].release(); p->dims[1].release();
     if (p->ev_maps) cudaEventDestroy(p->ev_maps);
     for (int b = 0; b < 2; ++b) if (p->ev_ld[b]) cudaEventDestroy(p->ev_ld[b]);
     for (int b = 0; b < 2; ++b) {
@@ -845,11 +907,19 @@ static int enqueue_assemble_and_fetch(b200pose_post* p, int n, cudaStream_t st) 
     return 0;
 }
 
+// dims_hw (host, may be null): a ragged run, n low-resolution (h, w) pairs; image i's maps lie top-left in the h x w canvas
 static int post_run_dev(b200pose_post* p, const float* d_heat, const float* d_paf, int layout, int n, int h, int w,
-                        float thresh, cudaStream_t st) {
+                        float thresh, cudaStream_t st, const int* dims_hw = nullptr) {
     if (n > p->pb.batch_cap) return fail("batch %d exceeds post batch_cap %d", n, p->pb.batch_cap);
     cudaStream_t ps = st;       // the stream peaks / limbs run on
     const int slot = (int)(p->runs & 1);
+    const int2* d_dims = nullptr;
+    if (dims_hw) {      // per run-parity slot: run i-1's kernels on the second stream may still read the other one
+        CU(p->dims[slot].ensure(p->pb.batch_cap));
+        if (p->have_ld[slot]) CU(cudaStreamWaitEvent(st, p->ev_ld[slot], 0));   // run i-2 is done with this slot
+        CU(cudaMemcpyAsync(p->dims[slot].p, dims_hw, (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, st));
+        d_dims = p->dims[slot].p;
+    }
     if (p->overlap) {
         // private copy of the maps (15 MB at batch 32) so that the next forward may overwrite the network's output
         // buffers while this run's post-processing is still reading; everything after the copy runs on s2
@@ -870,10 +940,11 @@ static int post_run_dev(b200pose_post* p, const float* d_heat, const float* d_pa
     if (p->runs > 0) CU(cudaStreamWaitEvent(ps, p->ev_fetch[(p->runs - 1) & 1], 0));
     cudaError_t e;
     if (layout == 0) {
-        e = post_peaks(p->pb, n, d_heat, (long)19 * h * w, (long)h * w, w, 1, h, w, thresh, ps);
+        e = post_peaks(p->pb, n, d_heat, (long)19 * h * w, (long)h * w, w, 1, h, w, thresh, ps, d_dims);
         if (e != cudaSuccess) return fail("post_peaks: %s", cudaGetErrorString(e));
-        e = post_limbs(p->pb, n, d_paf, (long)38 * h * w, (long)h * w, w, 1, 3, h * 8, w, h, ps);
+        e = post_limbs(p->pb, n, d_paf, (long)38 * h * w, (long)h * w, w, 1, 3, h * 8, w, h, ps, d_dims);
     } else {
+        if (d_dims) return fail("ragged runs take NCHW maps");
         e = post_peaks(p->pb, n, d_heat, (long)19 * h * w, 1, (long)w * 19, 19, h, w, thresh, ps);
         if (e != cudaSuccess) return fail("post_peaks: %s", cudaGetErrorString(e));
         e = post_limbs(p->pb, n, d_paf, (long)38 * h * w, 1, (long)w * 38, 38, 3, h * 8, w, h, ps);
@@ -1201,6 +1272,77 @@ int b200pose_infer_raw_u8(b200pose_net* net, b200pose_post* post, const unsigned
                         w, post->d_heat.p, post->d_paf.p, st);
     if (rc) return rc;
     return post_run_dev(post, post->d_heat.p, post->d_paf.p, 0, n, h, w, thresh, st);
+}
+
+// Per-frame geometry of a ragged batch of raw frames packed back to back: crop_with_factor of each frame's own size,
+// its byte offset in the packed input, and the canvas (largest padded height x largest padded width).
+static int ragged_layout(int n, const int* src_h, const int* src_w, int dest_size, int factor, RaggedCrop* fr,
+                         int* canvas_h, int* canvas_w) {
+    if (!src_h || !src_w) return fail("ragged layout: null pointer");
+    if (n < 1) return fail("ragged layout: no frames");
+    int H = 0, W = 0;
+    long off = 0;
+    for (int i = 0; i < n; ++i) {
+        if (int rc = crop_check(1, src_h[i], src_w[i], dest_size, factor, &fr[i].g)) {
+            fail("ragged layout: frame %d (%d x %d): %s", i, src_h[i], src_w[i], g_err.c_str());
+            return rc;
+        }
+        fr[i].src_off = off; fr[i].src_h = src_h[i]; fr[i].src_w = src_w[i];
+        off += (long)src_h[i] * src_w[i] * 3;
+        H = H > fr[i].g.pad_h ? H : fr[i].g.pad_h;
+        W = W > fr[i].g.pad_w ? W : fr[i].g.pad_w;
+    }
+    if ((long)H * W > (1L << 28)) return fail("ragged layout: canvas %d x %d too large", H, W);
+    *canvas_h = H;
+    *canvas_w = W;
+    return 0;
+}
+
+int b200pose_ragged_layout(int n, const int* src_h, const int* src_w, int dest_size, int factor, long* src_off,
+                           int* pad_h, int* pad_w, int* canvas_h, int* canvas_w) {
+    if (!src_off || !pad_h || !pad_w || !canvas_h || !canvas_w) return fail("ragged layout: null pointer");
+    std::vector<RaggedCrop> fr(n > 0 ? n : 0);
+    if (int rc = ragged_layout(n, src_h, src_w, dest_size, factor, fr.data(), canvas_h, canvas_w)) return rc;
+    for (int i = 0; i < n; ++i) { src_off[i] = fr[i].src_off; pad_h[i] = fr[i].g.pad_h; pad_w[i] = fr[i].g.pad_w; }
+    return 0;
+}
+
+int b200pose_infer_raw_u8_ragged(b200pose_net* net, b200pose_post* post, const unsigned char* frames,
+                                 int input_on_device, int n, const int* src_h, const int* src_w, int dest_size,
+                                 int factor, int mode, float thresh, void* cuda_stream) {
+    if (!net || !post) return fail("null handle");
+    if (!net->finalized) return fail("net not finalized");
+    if (net->device != post->device) return fail("net and post live on different devices");
+    if (!frames || !src_h || !src_w) return fail("infer_raw_ragged: null pointer");
+    if (n < 1) return fail("infer_raw_ragged: no frames");
+    if (n > post->pb.batch_cap) return fail("batch %d exceeds post batch_cap %d", n, post->pb.batch_cap);
+    std::vector<RaggedCrop> fr(n);
+    std::vector<int> ext_h(n), ext_w(n), dims(2 * n);
+    int H = 0, W = 0;
+    if (int rc = ragged_layout(n, src_h, src_w, dest_size, factor, fr.data(), &H, &W)) return rc;
+    for (int i = 0; i < n; ++i) {
+        ext_h[i] = fr[i].g.pad_h; ext_w[i] = fr[i].g.pad_w;
+        dims[2 * i] = fr[i].g.pad_h / 8; dims[2 * i + 1] = fr[i].g.pad_w / 8;
+    }
+    const long off = fr[n - 1].src_off + (long)src_h[n - 1] * src_w[n - 1] * 3;     // bytes of the packed frames
+    CU(cudaSetDevice(net->device));
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(cuda_stream);
+    // the caller keeps a host input alive until b200pose_post_sync(), as for b200pose_infer_raw_u8
+    const unsigned char* d_raw = frames;
+    if (!input_on_device) {
+        CU(net->raw_stage.ensure(off));
+        CU(cudaMemcpyAsync(net->raw_stage.p, frames, off, cudaMemcpyHostToDevice, st));
+        d_raw = net->raw_stage.p;
+    }
+    CU(net->rcrop.ensure(n));
+    CU(cudaMemcpyAsync(net->rcrop.p, fr.data(), n * sizeof(RaggedCrop), cudaMemcpyHostToDevice, st));
+    CU(net->in_stage_u8.ensure((size_t)n * H * W * 3));
+    cudaError_t e = crop_with_factor_ragged_launch(d_raw, net->in_stage_u8.p, n, net->rcrop.p, H, W, st);
+    if (e != cudaSuccess) return fail("crop_with_factor_ragged_launch: %s", cudaGetErrorString(e));
+    ++g_launches;
+    int rc = net_forward_impl(net, net->in_stage_u8.p, 1, 1, n, H, W, mode, nullptr, 1, st, false, ext_h.data(), ext_w.data());
+    if (rc) return rc;
+    return post_run_dev(post, net->out_f32[11].p, net->out_f32[10].p, 0, n, H / 8, W / 8, thresh, st, dims.data());
 }
 
 int b200pose_infer_raw_u8_multiscale(b200pose_net* net, b200pose_post* post, const unsigned char* images,

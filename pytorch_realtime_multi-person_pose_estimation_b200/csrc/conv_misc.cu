@@ -29,12 +29,15 @@ template <int kIn>
 __global__ void __launch_bounds__(kF_Threads) conv_first_kernel(const void* __restrict__ in_v, const float* __restrict__ wgt,
                                                                 const float* __restrict__ bias,
                                                                 __nv_bfloat16* __restrict__ out,
-                                                                __nv_bfloat16* __restrict__ out_lo, int H, int W) {
+                                                                __nv_bfloat16* __restrict__ out_lo, int H, int W,
+                                                                const int2* __restrict__ ext) {
     constexpr bool kU8 = kIn != 0;
     __shared__ float s_in[3][kF_TH + 2][kF_TW + 2];
     __shared__ __align__(16) float s_w[27][64];
     __shared__ float s_b[64];
     const int n = blockIdx.z, y0 = blockIdx.y * kF_TH, x0 = blockIdx.x * kF_TW;
+    // ragged batches: the image's extent in its canvas slot; pixels beyond it are the conv's zero padding
+    const int2 e = ext != nullptr ? ext[n] : make_int2(H, W);
     const int tid = threadIdx.x;
     for (int i = tid; i < 27 * 64; i += kF_Threads) {
         // wgt is OIHW [64][3][3][3]; s_w[(c*3+ky)*3+kx][o]
@@ -57,7 +60,7 @@ __global__ void __launch_bounds__(kF_Threads) conv_first_kernel(const void* __re
         }
         const int gy = y0 + yy - 1, gx = x0 + xx - 1;
         float v = 0.f;
-        if (gy >= 0 && gy < H && gx >= 0 && gx < W) {
+        if (gy >= 0 && gy < e.x && gx >= 0 && gx < e.y) {
             if (kU8) {
                 const unsigned char u =
                     static_cast<const unsigned char*>(in_v)[(((size_t)n * H + gy) * W + gx) * 3 + pre_src_channel(kIn, c)];
@@ -105,6 +108,10 @@ __global__ void __launch_bounds__(kF_Threads) conv_first_kernel(const void* __re
 #pragma unroll
             for (int p = 0; p < 2; ++p) {
                 if (x + p >= W) continue;
+                if (y >= e.x || x + p >= e.y) {      // outside the image's extent: +0
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) acc[p][j] = 0.f;
+                }
                 __nv_bfloat16* dst = out + (((size_t)n * H + y) * W + x + p) * 64 + o0;
                 uint32_t pk[8];
 #pragma unroll
@@ -154,12 +161,14 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 template <int kIn>
 __global__ void __launch_bounds__(kF_Threads) conv_first_mma_kernel(const void* __restrict__ in_v, const float* __restrict__ wgt,
                                                                     const float* __restrict__ bias,
-                                                                    __nv_bfloat16* __restrict__ out, int H, int W) {
+                                                                    __nv_bfloat16* __restrict__ out, int H, int W,
+                                                                    const int2* __restrict__ ext) {
     constexpr bool kU8 = kIn != 0;
     constexpr int kRowF = kF_TW + 2, kPlaneF = (kF_TH + 2) * kRowF;
     __shared__ float s_in[3 * kPlaneF];
     __shared__ __align__(16) uint32_t s_out[kF_TH * kF_TW * 32];      // [pixel][8 chunks of 16 B], chunk index ^ (pixel & 7)
     const int n = blockIdx.z, y0 = blockIdx.y * kF_TH, x0 = blockIdx.x * kF_TW;
+    const int2 e = ext != nullptr ? ext[n] : make_int2(H, W);          // ragged batches: the image's extent
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int i = tid; i < 3 * kPlaneF; i += kF_Threads) {
         int c, yy, xx;
@@ -176,7 +185,7 @@ __global__ void __launch_bounds__(kF_Threads) conv_first_mma_kernel(const void* 
         }
         const int gy = y0 + yy - 1, gx = x0 + xx - 1;
         float v = 0.f;
-        if (gy >= 0 && gy < H && gx >= 0 && gx < W) {
+        if (gy >= 0 && gy < e.x && gx >= 0 && gx < e.y) {
             if (kU8) {
                 const unsigned char u =
                     static_cast<const unsigned char*>(in_v)[(((size_t)n * H + gy) * W + gx) * 3 + pre_src_channel(kIn, c)];
@@ -248,7 +257,7 @@ __global__ void __launch_bounds__(kF_Threads) conv_first_mma_kernel(const void* 
         const int y = y0 + p / kF_TW, x = x0 + p % kF_TW;
         if (y < H && x < W)
             reinterpret_cast<uint4*>(out + (((size_t)n * H + y) * W + x) * 64)[ch] =
-                reinterpret_cast<const uint4*>(s_out + p * 32)[ch ^ (p & 7)];
+                (y < e.x && x < e.y) ? reinterpret_cast<const uint4*>(s_out + p * 32)[ch ^ (p & 7)] : make_uint4(0, 0, 0, 0);
     }
 }
 
@@ -313,12 +322,14 @@ __global__ void __launch_bounds__(kR_Threads) conv_f32_kernel(ConvF32Args a) {
         const int p = pg * 4 + i;
         const int y = ty0 + (p >> 3), x = tx0 + (p & 7);
         if (y >= a.H || x >= a.W) continue;
+        const bool zero = a.ext != nullptr && (y >= (a.ext[n].x >> a.ext_shift) || x >= (a.ext[n].y >> a.ext_shift));
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int o = co0 + cg * 4 + j;
             if (o >= a.cout) continue;
             float v = acc[i][j] + a.bias[o];
             if (a.relu) v = fmaxf(v, 0.f);
+            if (zero) v = 0.f;          // ragged batches: outside the image's extent
             a.out[(((size_t)n * a.H + y) * a.W + x) * a.out_cstride + a.out_ch_off + o] = v;
             if (a.out_nchw) a.out_nchw[(((size_t)n * a.cout + o) * a.H + y) * a.W + x] = v;
         }
@@ -357,25 +368,26 @@ __global__ void nchw_to_nhwc_f32_kernel(const float* __restrict__ in, float* __r
 }  // namespace
 
 cudaError_t conv_first_launch(const void* in, int in_is_u8_hwc, const float* w_oihw, const float* bias,
-                              __nv_bfloat16* out_nhwc, __nv_bfloat16* out_lo, int N, int H, int W, cudaStream_t s) {
+                              __nv_bfloat16* out_nhwc, __nv_bfloat16* out_lo, int N, int H, int W, cudaStream_t s,
+                              const int2* ext) {
     dim3 grid((W + kF_TW - 1) / kF_TW, (H + kF_TH - 1) / kF_TH, N);
     if (out_lo == nullptr) {        // bf16 mode: tensor cores
         switch (in_is_u8_hwc) {
-            case kPreNone: conv_first_mma_kernel<kPreNone><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W); break;
-            case kPreRtpose: conv_first_mma_kernel<kPreRtpose><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W); break;
-            case kPreVgg: conv_first_mma_kernel<kPreVgg><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W); break;
-            case kPreInception: conv_first_mma_kernel<kPreInception><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W); break;
-            case kPreSsd: conv_first_mma_kernel<kPreSsd><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W); break;
+            case kPreNone: conv_first_mma_kernel<kPreNone><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W, ext); break;
+            case kPreRtpose: conv_first_mma_kernel<kPreRtpose><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W, ext); break;
+            case kPreVgg: conv_first_mma_kernel<kPreVgg><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W, ext); break;
+            case kPreInception: conv_first_mma_kernel<kPreInception><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W, ext); break;
+            case kPreSsd: conv_first_mma_kernel<kPreSsd><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, H, W, ext); break;
             default: return cudaErrorInvalidValue;
         }
         return cudaGetLastError();
     }
     switch (in_is_u8_hwc) {
-        case kPreNone: conv_first_kernel<kPreNone><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W); break;
-        case kPreRtpose: conv_first_kernel<kPreRtpose><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W); break;
-        case kPreVgg: conv_first_kernel<kPreVgg><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W); break;
-        case kPreInception: conv_first_kernel<kPreInception><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W); break;
-        case kPreSsd: conv_first_kernel<kPreSsd><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W); break;
+        case kPreNone: conv_first_kernel<kPreNone><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W, ext); break;
+        case kPreRtpose: conv_first_kernel<kPreRtpose><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W, ext); break;
+        case kPreVgg: conv_first_kernel<kPreVgg><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W, ext); break;
+        case kPreInception: conv_first_kernel<kPreInception><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W, ext); break;
+        case kPreSsd: conv_first_kernel<kPreSsd><<<grid, kF_Threads, 0, s>>>(in, w_oihw, bias, out_nhwc, out_lo, H, W, ext); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -383,7 +395,7 @@ cudaError_t conv_first_launch(const void* in, int in_is_u8_hwc, const float* w_o
 
 namespace {
 __global__ void u8hwc_to_f32nchw_kernel(const unsigned char* __restrict__ in, float* __restrict__ out, int N, int H, int W,
-                                        int mode) {
+                                        int mode, const int2* __restrict__ ext) {
     const size_t total = (size_t)N * 3 * H * W;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const int x = i % W;
@@ -392,16 +404,18 @@ __global__ void u8hwc_to_f32nchw_kernel(const unsigned char* __restrict__ in, fl
         t /= H;
         const int c = t % 3;
         const int n = t / 3;
-        out[i] = pre_value(mode, in[(((size_t)n * H + y) * W + x) * 3 + pre_src_channel(mode, c)], c);
+        if (ext != nullptr && (y >= ext[n].x || x >= ext[n].y)) out[i] = 0.f;     // outside a ragged image: conv padding
+        else out[i] = pre_value(mode, in[(((size_t)n * H + y) * W + x) * 3 + pre_src_channel(mode, c)], c);
     }
 }
 }  // namespace
 
-cudaError_t u8hwc_to_f32nchw_launch(const unsigned char* in, float* out, int N, int H, int W, int mode, cudaStream_t s) {
+cudaError_t u8hwc_to_f32nchw_launch(const unsigned char* in, float* out, int N, int H, int W, int mode, cudaStream_t s,
+                                    const int2* ext) {
     if (mode < kPreRtpose || mode > kPreSsd) return cudaErrorInvalidValue;
     const size_t total = (size_t)N * 3 * H * W;
     const int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
-    u8hwc_to_f32nchw_kernel<<<blocks, 256, 0, s>>>(in, out, N, H, W, mode);
+    u8hwc_to_f32nchw_kernel<<<blocks, 256, 0, s>>>(in, out, N, H, W, mode, ext);
     return cudaGetLastError();
 }
 

@@ -72,6 +72,14 @@ __device__ __forceinline__ TileCoord decode_tile(int t, int n_tiles, int groups,
     return c;
 }
 
+// Ragged batches (a.ext): input-resolution pixel (y, x) of image n lies outside that image's extent.  Extents are multiples
+// of 8 and pooled layers have ext_shift <= 2, so a 2x2 pooling window lies wholly inside or wholly outside.
+__device__ __forceinline__ bool outside_extent(const ConvTcArgs& a, int n, int y, int x) {
+    if (a.ext == nullptr) return false;
+    const int2 e = __ldg(a.ext + n);
+    return y >= (e.x >> a.ext_shift) || x >= (e.y >> a.ext_shift);
+}
+
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&v);
@@ -392,6 +400,7 @@ __device__ __forceinline__ void conv_tc_body(const ConvTcArgs& a) {
                         const int x = tc.x0 + sub * 8 + w_in;
                         const bool valid = tc.valid && (y < a.H) && (x < a.W);
                         const bool writer = a.pool ? (valid && !(lane & 1) && !(lane & 8)) : valid;
+                        const bool zero = valid && outside_extent(a, tc.n, y, x);
                         const int yo = a.pool ? y >> 1 : y;
                         const int xo = a.pool ? x >> 1 : x;
                         float v[32];
@@ -400,6 +409,7 @@ __device__ __forceinline__ void conv_tc_body(const ConvTcArgs& a) {
                             const float bj = (full || j < 16) ? __ldg(bias + c0 + j) : 0.f;
                             v[j] = accr[sub][j] + bj;
                             if (a.relu) v[j] = fmaxf(v[j], 0.f);
+                            if (zero) v[j] = 0.f;
                         }
                         if (a.pool) {
 #pragma unroll
@@ -464,6 +474,7 @@ __device__ __forceinline__ void conv_tc_body(const ConvTcArgs& a) {
                 const bool valid = tc.valid && (y < a.H) && (x < a.W);
                 // pooled: lanes with even (h, w) own the 2x2 window
                 const bool writer = a.pool ? (valid && !(lane & 1) && !(lane & 8)) : valid;
+                const bool zero = valid && outside_extent(a, tc.n, y, x);
                 const int yo = a.pool ? y >> 1 : y;
                 const int xo = a.pool ? x >> 1 : x;
                 const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + ai * 256 + sub * 128;
@@ -494,6 +505,7 @@ __device__ __forceinline__ void conv_tc_body(const ConvTcArgs& a) {
                     for (int j = 0; j < 32; ++j) {
                         v[j] = __uint_as_float(r[j]) + bv[j];
                         if (a.relu) v[j] = fmaxf(v[j], 0.f);
+                        if (zero) v[j] = 0.f;
                     }
                     if (a.pool) {
 #pragma unroll

@@ -65,6 +65,12 @@ struct ConvTcArgs {
     int tps;
     // ---- programmatic dependent launch of this layer behind the previous one (small-batch plans)
     int pdl;
+    // ---- ragged batches: full-resolution (h, w) of every image, the image sitting top-left in its slot of the [H, W]
+    //      canvas; output pixels outside (h >> ext_shift, w >> ext_shift) at this layer's input resolution store zeros
+    //      (bf16, residual plane and fp32 copy), so that the next layer's halo reads what TMA's zero fill gives the image
+    //      alone.  nullptr: every image fills the canvas.
+    const int2* ext;
+    int ext_shift;
     // ---- tensor maps
     CUtensorMap tm_in;        // 4D (C, W, H, N) bf16, box (64, 24, 16+ks-1, 1), SWIZZLE_128B
     CUtensorMap tm_w;         // 3D (cin_pad, groups*n_tiles*n_tile, 2*taps) bf16 [hi taps | lo taps], box (64, n_tile, tps)

@@ -165,7 +165,8 @@ struct PlanePaf {          // the limb's two PAF planes in shared memory: channe
 };
 
 __global__ void __launch_bounds__(kScoreThreads) limb_score_kernel(PostBuffers pb, PafView paf0, long p_img, int h_up,
-                                                                   int lw, int lh, int paf_in_smem, int n_limbs) {
+                                                                   int lw, int lh, int paf_in_smem, int n_limbs,
+                                                                   const int2* __restrict__ dims) {
     extern __shared__ float s_planes[];
     __shared__ int s_item;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -196,6 +197,7 @@ __global__ void __launch_bounds__(kScoreThreads) limb_score_kernel(PostBuffers p
         const LimbPlan pl = pb.lplan[li];
         const int img = li / kNumLimb, limb = li - img * kNumLimb;
         const int chunk = item - pl.work0;
+        const int img_h_up = dims != nullptr ? 8 * dims[img].x : h_up;     // ragged batch: the image's own padded height
         const int pa = c_lparts[limb][0], pbp = c_lparts[limb][1];
         const int c1 = c_lpaf[limb][0], c2 = c_lpaf[limb][1];
         PafView paf = paf0;
@@ -234,8 +236,8 @@ __global__ void __launch_bounds__(kScoreThreads) limb_score_kernel(PostBuffers p
                 bool pass = false;
                 if (p < npairs) {
                     const int ax = __ldg(axp + a), ay = __ldg(ayp + a), bx = __ldg(bxp + b), by = __ldg(byp + b);
-                    pass = paf_in_smem ? pair_score_t(pp, 0, 1, ax, ay, bx, by, h_up, &sc)
-                                       : pair_score_t(paf, c1, c2, ax, ay, bx, by, h_up, &sc);
+                    pass = paf_in_smem ? pair_score_t(pp, 0, 1, ax, ay, bx, by, img_h_up, &sc)
+                                       : pair_score_t(paf, c1, c2, ax, ay, bx, by, img_h_up, &sc);
                 }
                 const unsigned m = __ballot_sync(0xffffffffu, pass);
                 if (pass) dst[cnt + __popc(m & lt)] = cand_key(sc, (uint32_t)p);
@@ -808,7 +810,7 @@ __global__ void __launch_bounds__(kGreedyThreads) limb_greedy_kernel(PostBuffers
     } while (0)
 
 cudaError_t post_limbs(const PostBuffers& pb, int batch, const float* paf, long p_img, long p_ch, long p_y, long p_x,
-                       int shift, int h_up, int lw, int lh, cudaStream_t s) {
+                       int shift, int h_up, int lw, int lh, cudaStream_t s, const int2* dims) {
     if (batch > pb.batch_cap) return cudaErrorInvalidValue;
     if (pb.cand_smem_cap != kS) return cudaErrorInvalidValue;
     PafView pv{paf, p_ch, p_y, p_x, shift};
@@ -825,7 +827,7 @@ cudaError_t post_limbs(const PostBuffers& pb, int batch, const float* paf, long 
     int dev = 0, sms = 148;
     B2P_TRY(cudaGetDevice(&dev));
     B2P_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    limb_score_kernel<<<sms * 6, kScoreThreads, smem, s>>>(pb, pv, p_img, h_up, lw, lh, in_smem, batch * kNumLimb);
+    limb_score_kernel<<<sms * 6, kScoreThreads, smem, s>>>(pb, pv, p_img, h_up, lw, lh, in_smem, batch * kNumLimb, dims);
     B2P_TRY(cudaGetLastError());
     limb_gather_kernel<<<dim3(batch, kNumLimb), kGatherThreads, 0, s>>>(pb);
     B2P_TRY(cudaGetLastError());

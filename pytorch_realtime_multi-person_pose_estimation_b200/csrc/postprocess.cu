@@ -100,8 +100,13 @@ __device__ __forceinline__ void refine_interior_slots(const float* plane, int w,
 }
 
 __global__ void __launch_bounds__(kPeakThreads, 512 / kPeakThreads) peaks_kernel(PostBuffers pb, const float* __restrict__ heat, long h_img,
-                                                             long h_ch, long h_y, long h_x, int h, int w, float thresh) {
+                                                             long h_ch, long h_y, long h_x, int h, int w, float thresh,
+                                                             const int2* __restrict__ dims) {
     extern __shared__ float sm_f[];
+    if (dims != nullptr) {      // ragged batch: this image's own map size (its plane sits top-left in the canvas strides)
+        h = dims[blockIdx.y].x;
+        w = dims[blockIdx.y].y;
+    }
     float* plane = sm_f;                       // [h*w]
     float* hor_all = sm_f + h * w;             // [8 warps][5][40]
     __shared__ int warp_cnt[kPeakThreads / 32];
@@ -449,14 +454,14 @@ void post_free(PostBuffers& pb) {
 }
 
 cudaError_t post_peaks(const PostBuffers& pb, int batch, const float* heat, long h_img, long h_ch, long h_y, long h_x,
-                       int h, int w, float thresh, cudaStream_t s) {
+                       int h, int w, float thresh, cudaStream_t s, const int2* dims) {
     if (batch > pb.batch_cap) return cudaErrorInvalidValue;
     const size_t smem = ((size_t)h * w + (kPeakThreads / 32) * 5 * kHorStride) * sizeof(float);
     if (smem > 200 * 1024) return cudaErrorInvalidValue;
     static DynSmemOptIn optin;
     B2P_TRY(optin.ensure(peaks_kernel, smem));
     B2P_TRY(cudaMemsetAsync(pb.status, 0, batch * sizeof(int), s));
-    peaks_kernel<<<dim3(kNumPart, batch), kPeakThreads, smem, s>>>(pb, heat, h_img, h_ch, h_y, h_x, h, w, thresh);
+    peaks_kernel<<<dim3(kNumPart, batch), kPeakThreads, smem, s>>>(pb, heat, h_img, h_ch, h_y, h_x, h, w, thresh, dims);
     return cudaGetLastError();
 }
 

@@ -79,11 +79,14 @@ cudaError_t post_alloc(PostBuffers& pb, int batch_cap, int peak_cap, int human_c
 void post_free(PostBuffers& pb);
 
 // heat: fp32, value(img, part, y, x) = heat[img*h_img + part*h_ch + y*h_y + x*h_x]; low-res (h x w).
+// dims (ragged batches, device array or null): image i's own low-res (h, w), its maps top-left in the h x w canvas.
 cudaError_t post_peaks(const PostBuffers& pb, int batch, const float* heat, long h_img, long h_ch, long h_y, long h_x,
-                       int h, int w, float thresh, cudaStream_t s);
+                       int h, int w, float thresh, cudaStream_t s, const int2* dims = nullptr);
 // paf: fp32 view per image: base + img*p_img, strides (p_ch, p_y, p_x), shift (3: low-res, 0: already upsampled).
+// dims (ragged batches): image i's own low-res (h, w); its length criterion uses h_up = 8 h instead of h_up.
 cudaError_t post_limbs(const PostBuffers& pb, int batch, const float* paf, long p_img, long p_ch, long p_y,
-                                    long p_x, int shift, int h_up, int lw, int lh, cudaStream_t s);
+                                    long p_x, int shift, int h_up, int lw, int lh, cudaStream_t s,
+                                    const int2* dims = nullptr);
 // Test hook (limbs.cu): exact std::sort of n host keys through the global-memory partition + shared-memory range kernels.
 cudaError_t post_debug_sort(const PostBuffers& pb, const unsigned long long* keys, int n, unsigned long long* out,
                             cudaStream_t s);

@@ -9,6 +9,28 @@ namespace {
 
 constexpr int kThreads = 256;
 
+// Destination pixel (y, x) of one frame: its three bytes, zero outside the resized area (the padding).
+__device__ __forceinline__ void crop_px3(const unsigned char* src, int src_h, int src_w, const CropGeom& g, int y, int x,
+                                         unsigned char* dst) {
+    unsigned char v0 = 0, v1 = 0, v2 = 0;
+    if (y < g.res_h && x < g.res_w) {
+        const long stride = (long)src_w * 3;
+        if (g.area2) {
+            v0 = rs_area2_px(src, src_h, src_w, stride, 3, 0, x, y);
+            v1 = rs_area2_px(src, src_h, src_w, stride, 3, 1, x, y);
+            v2 = rs_area2_px(src, src_h, src_w, stride, 3, 2, x, y);
+        } else {
+            const LinCoef cx = rs_coef_x(x, src_w, g.step), cy = rs_coef_y(y, src_h, g.step);
+            v0 = rs_linear_px(src, stride, 3, 0, cx, cy);
+            v1 = rs_linear_px(src, stride, 3, 1, cx, cy);
+            v2 = rs_linear_px(src, stride, 3, 2, cx, cy);
+        }
+    }
+    dst[0] = v0;
+    dst[1] = v1;
+    dst[2] = v2;
+}
+
 __global__ void __launch_bounds__(kThreads) crop_with_factor_kernel(const unsigned char* __restrict__ in,
                                                                     unsigned char* __restrict__ out, int src_h, int src_w,
                                                                     CropGeom g) {
@@ -18,23 +40,24 @@ __global__ void __launch_bounds__(kThreads) crop_with_factor_kernel(const unsign
     unsigned char* dst = out + img * dst_px * 3;
     for (long p = blockIdx.x * (long)kThreads + threadIdx.x; p < dst_px; p += (long)gridDim.x * kThreads) {
         const int y = (int)(p / g.pad_w), x = (int)(p - (long)y * g.pad_w);
-        unsigned char v0 = 0, v1 = 0, v2 = 0;
-        if (y < g.res_h && x < g.res_w) {
-            const long stride = (long)src_w * 3;
-            if (g.area2) {
-                v0 = rs_area2_px(src, src_h, src_w, stride, 3, 0, x, y);
-                v1 = rs_area2_px(src, src_h, src_w, stride, 3, 1, x, y);
-                v2 = rs_area2_px(src, src_h, src_w, stride, 3, 2, x, y);
-            } else {
-                const LinCoef cx = rs_coef_x(x, src_w, g.step), cy = rs_coef_y(y, src_h, g.step);
-                v0 = rs_linear_px(src, stride, 3, 0, cx, cy);
-                v1 = rs_linear_px(src, stride, 3, 1, cx, cy);
-                v2 = rs_linear_px(src, stride, 3, 2, cx, cy);
-            }
-        }
-        dst[3 * p + 0] = v0;
-        dst[3 * p + 1] = v1;
-        dst[3 * p + 2] = v2;
+        crop_px3(src, src_h, src_w, g, y, x, dst + 3 * p);
+    }
+}
+
+// Ragged batch: frame i (its own source size and geometry) fills slot i of the [n, canvas_h, canvas_w, 3] canvas from the
+// top-left corner; everything beyond its resized area - its padding and the rest of the slot - is zero.
+__global__ void __launch_bounds__(kThreads) crop_with_factor_ragged_kernel(const unsigned char* __restrict__ in,
+                                                                           unsigned char* __restrict__ out,
+                                                                           const RaggedCrop* __restrict__ frames,
+                                                                           int canvas_h, int canvas_w) {
+    const int img = blockIdx.y;
+    const RaggedCrop f = frames[img];
+    const long dst_px = (long)canvas_h * canvas_w;
+    const unsigned char* src = in + f.src_off;
+    unsigned char* dst = out + img * dst_px * 3;
+    for (long p = blockIdx.x * (long)kThreads + threadIdx.x; p < dst_px; p += (long)gridDim.x * kThreads) {
+        const int y = (int)(p / canvas_w), x = (int)(p - (long)y * canvas_w);
+        crop_px3(src, f.src_h, f.src_w, f.g, y, x, dst + 3 * p);
     }
 }
 
@@ -77,6 +100,18 @@ cudaError_t crop_with_factor_launch(const unsigned char* in, unsigned char* out,
     if (bx > cap) bx = cap;
     if (bx < 1) bx = 1;
     crop_with_factor_kernel<<<dim3((unsigned)bx, (unsigned)n), kThreads, 0, s>>>(in, out, src_h, src_w, g);
+    return cudaGetLastError();
+}
+
+cudaError_t crop_with_factor_ragged_launch(const unsigned char* in, unsigned char* out, int n, const RaggedCrop* frames,
+                                           int canvas_h, int canvas_w, cudaStream_t s) {
+    if (n < 1 || n > 65535 || canvas_h < 1 || canvas_w < 1) return cudaErrorInvalidValue;
+    const long px = (long)canvas_h * canvas_w;
+    long bx = (px + kThreads - 1) / kThreads;
+    const long cap = (148L * 8 + n - 1) / n;
+    if (bx > cap) bx = cap;
+    if (bx < 1) bx = 1;
+    crop_with_factor_ragged_kernel<<<dim3((unsigned)bx, (unsigned)n), kThreads, 0, s>>>(in, out, frames, canvas_h, canvas_w);
     return cudaGetLastError();
 }
 

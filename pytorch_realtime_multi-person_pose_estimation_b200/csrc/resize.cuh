@@ -12,6 +12,17 @@ namespace b2p {
 cudaError_t crop_with_factor_launch(const unsigned char* in, unsigned char* out, int n, int src_h, int src_w,
                                     const CropGeom& g, cudaStream_t s);
 
+// Ragged batch of raw frames of different sizes, packed back to back: frame i starts at byte src_off and has its own
+// geometry (crop_geometry of its size).  out [n, canvas_h, canvas_w, 3]: frame i resized and padded exactly as
+// crop_with_factor_launch does it, in the top-left corner of slot i, zeros elsewhere.  `frames` is a device array.
+struct RaggedCrop {
+    CropGeom g;
+    long src_off;
+    int src_h, src_w;
+};
+cudaError_t crop_with_factor_ragged_launch(const unsigned char* in, unsigned char* out, int n, const RaggedCrop* frames,
+                                           int canvas_h, int canvas_w, cudaStream_t s);
+
 // Bicubic resize of `planes` float32 planes [src_h, src_w] -> [dst_h, dst_w] (resize_core.h: rs_cubic_at), fused with
 // the running sum of the multi-scale average: dst = first ? r : dst + r, then dst /= divide_by when divide_by > 0.
 cudaError_t resize_cubic_accum_launch(const float* src, float* dst, long planes, int src_h, int src_w, int dst_h,

@@ -47,6 +47,18 @@ class NativeNet:
                                                     arr, int(out_on_device), ctypes.c_void_p(stream)),
                   "b200pose_net_forward_u8")
 
+    def forward_u8_ragged_ptr(self, in_ptr, in_on_device, n, H, W, ext_h, ext_w, mode, out_ptrs, out_on_device, stream):
+        """Ragged batch: uint8 HWC BGR canvas [n,H,W,3], frame i valid in its top-left ext_h[i] x ext_w[i] (multiples of
+        8); outputs canvas-shaped, +0 outside each extent, bit-identical to forward_u8_ptr of each frame alone inside."""
+        if len(ext_h) != n or len(ext_w) != n:
+            raise nat.B200PoseError("forward_u8_ragged_ptr: %d images but %d / %d extents" % (n, len(ext_h), len(ext_w)))
+        arr = (ctypes.c_void_p * 12)(*[ctypes.c_void_p(p) if p else None for p in out_ptrs])
+        eh = (ctypes.c_int * n)(*[int(v) for v in ext_h])
+        ew = (ctypes.c_int * n)(*[int(v) for v in ext_w])
+        nat.check(nat.lib().b200pose_net_forward_u8_ragged(self._h, ctypes.c_void_p(in_ptr), int(in_on_device), n, H, W,
+                                                           eh, ew, mode, arr, int(out_on_device), ctypes.c_void_p(stream)),
+                  "b200pose_net_forward_u8_ragged")
+
     def crop_with_factor(self, images, dest_size=368, factor=8):
         """Device-side crop_with_factor (im_transform.py:119-134) of uint8 BGR frames of one size: [n,h,w,3] or [h,w,3]
         -> (padded frames, im_scale, resized shape) like the reference (which returns them for one image)."""
@@ -187,6 +199,29 @@ def humans_to_dicts(rows, width, height):
     return out
 
 
+def _of_image(v, i):
+    """Padded size of image i of a run: runs of one shape keep an int, ragged runs a tuple per image."""
+    return v[i] if isinstance(v, tuple) else v
+
+
+def ragged_groups(padded_shapes, batch_cap):
+    """Frames of different padded sizes [(ph, pw), ...] -> ragged runs: a list of (frame indices, (canvas_h, canvas_w)).
+    Landscape (ph <= pw) and portrait frames go to separate runs: the short side is dest_size for both, so a run's canvas
+    only wastes pixels along the long side.  Each orientation is sorted by the padded long side (ties in input order) and
+    cut into runs of at most batch_cap frames; the canvas of a run is the largest ph x the largest pw of its frames."""
+    if batch_cap < 1:
+        raise nat.B200PoseError("ragged_groups: batch_cap must be >= 1")
+    shapes = [(int(h), int(w)) for h, w in padded_shapes]
+    land = sorted((i for i, (h, w) in enumerate(shapes) if h <= w), key=lambda i: (shapes[i][1], i))
+    port = sorted((i for i, (h, w) in enumerate(shapes) if h > w), key=lambda i: (shapes[i][0], i))
+    runs = []
+    for idx in (land, port):
+        for k in range(0, len(idx), batch_cap):
+            part = idx[k:k + batch_cap]
+            runs.append((part, (max(shapes[i][0] for i in part), max(shapes[i][1] for i in part))))
+    return runs
+
+
 class PoseEngine:
     """Fused batched inference on one GPU: images -> humans, maps never leave the device."""
 
@@ -203,7 +238,8 @@ class PoseEngine:
 
     def _remember(self, n, H, W):
         """Shape of the run just submitted, kept per ticket (two runs may be in flight with different batch sizes or
-        frame shapes: fetch(ticket=i) must read run i with run i's n and normalise by run i's W / H)."""
+        frame shapes: fetch(ticket=i) must read run i with run i's n and normalise image k by run i's W[k] / H[k]).
+        H, W: one padded size for the whole run, or per-image tuples (ragged runs)."""
         t = self.post.last_ticket()
         if self.__dict__.get("_shapes") is None:
             self._shapes = {}
@@ -279,6 +315,34 @@ class PoseEngine:
         _, _, (ph, pw) = nat.crop_geometry(src_h, src_w, dest_size, factor)
         return self._remember(n, ph, pw)
 
+    def infer_raw_ragged_async_u8(self, frames, dest_size=368, factor=8, thresh=0.1, stream=0):
+        """Raw uint8 BGR frames of DIFFERENT sizes (a list of [h,w,3] arrays, at most batch_cap): every frame gets its own
+        crop_with_factor, then all of them run through the network and the post-processing as one batch (a canvas of the
+        largest padded height x width).  Returns a ticket; per frame the person rows equal infer_raw_async_u8 of that frame
+        alone, coordinates in pixels of its own padded frame."""
+        frames = [np.ascontiguousarray(f) for f in frames]
+        if not frames:
+            raise nat.B200PoseError("infer_raw_ragged_async_u8: no frames")
+        for f in frames:
+            if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3:
+                raise nat.B200PoseError("infer_raw_ragged_async_u8: expected uint8 [h,w,3] frames")
+        n = len(frames)
+        packed = np.concatenate([f.reshape(-1) for f in frames])
+        sh = (ctypes.c_int * n)(*[f.shape[0] for f in frames])
+        sw = (ctypes.c_int * n)(*[f.shape[1] for f in frames])
+        nat.check(nat.lib().b200pose_infer_raw_u8_ragged(self.net._h, self.post._h, ctypes.c_void_p(packed.ctypes.data), 0,
+                                                         n, sh, sw, int(dest_size), int(factor), self.mode,
+                                                         ctypes.c_float(thresh), ctypes.c_void_p(stream)),
+                  "b200pose_infer_raw_u8_ragged")
+        _, pads, _ = nat.ragged_layout([f.shape[:2] for f in frames], dest_size, factor)
+        t = self._remember(n, tuple(p[0] for p in pads), tuple(p[1] for p in pads))
+        if self.__dict__.get("_alive") is None:
+            self._alive = {}
+        self._alive[t] = packed                     # host staging is read asynchronously: keep it until the fetch
+        for old in [k for k in self._alive if k < t - 1]:
+            del self._alive[old]
+        return t
+
     def infer_raw_multiscale_async_u8(self, in_ptr, in_on_device, n, src_h, src_w, scales, base_size=368, factor=8,
                                       thresh=0.1, flip=False, stream=0):
         """Multi-scale (+ flip) test-time averaging of raw uint8 BGR frames of one size (BASELINE.json configs[4]):
@@ -294,21 +358,40 @@ class PoseEngine:
         _, _, (ph, pw) = nat.crop_geometry(src_h, src_w, base_size, factor)
         return self._remember(n, ph, pw)
 
-    def infer_images_arrays(self, images, dest_size=368, factor=8, thresh=0.1, flip=False, scales=None):
+    def infer_images_arrays(self, images, dest_size=368, factor=8, thresh=0.1, flip=False, scales=None, ragged=False):
         """infer_images, but per image the raw person rows (float32 [k, 73], pixel coordinates of the padded frame)."""
-        return self.infer_images(images, dest_size, factor, thresh, flip, scales, _arrays=True)
+        return self.infer_images(images, dest_size, factor, thresh, flip, scales, ragged, _arrays=True)
 
-    def infer_images(self, images, dest_size=368, factor=8, thresh=0.1, flip=False, scales=None, _arrays=False):
+    def infer_images(self, images, dest_size=368, factor=8, thresh=0.1, flip=False, scales=None, ragged=False,
+                     _arrays=False):
         """images: a list of raw uint8 BGR frames of arbitrary (mixed) sizes, as cv2.imread returns them.  Frames are
         bucketed by shape (one launch sequence per bucket, at most batch_cap frames each); returns per-image human lists
         in input order, coordinates normalised to the padded frame like paf_to_pose_cpp's.
-        scales: e.g. (0.5, 1.0, 1.5, 2.0) for multi-scale test-time averaging around dest_size."""
+        scales: e.g. (0.5, 1.0, 1.5, 2.0) for multi-scale test-time averaging around dest_size.
+        ragged=True: frames of different sizes share runs (ragged_groups: by orientation and padded long side, up to
+        batch_cap frames each; the next run is submitted before the previous one is fetched) - same results as the
+        bucketed path, fewer and fuller batches on photo collections.  Not combined with flip or scales."""
+        if ragged and (flip or scales is not None):
+            raise nat.B200PoseError("infer_images: ragged=True does not combine with flip or scales")
         buckets = {}
         for i, im in enumerate(images):
             if im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3:
                 raise nat.B200PoseError("infer_images: expected uint8 [h,w,3] frames")
             buckets.setdefault(im.shape[:2], []).append(i)
         out = [None] * len(images)
+        if ragged and images:
+            _, pads, _ = nat.ragged_layout([im.shape[:2] for im in images], dest_size, factor)
+            pending = None
+            for part, _ in ragged_groups(pads, self.post.batch_cap) + [(None, None)]:
+                t = None if part is None else self.infer_raw_ragged_async_u8([images[i] for i in part], dest_size, factor,
+                                                                              thresh)
+                if pending is not None:
+                    pt, pidx = pending
+                    res = self.fetch_arrays(ticket=pt) if _arrays else self.fetch(ticket=pt)
+                    for i, humans in zip(pidx, res):
+                        out[i] = humans.copy() if _arrays else humans
+                pending = None if part is None else (t, part)
+            return out
         for (sh, sw), idx in buckets.items():
             for k in range(0, len(idx), self.post.batch_cap):
                 part = idx[k:k + self.post.batch_cap]
@@ -332,7 +415,7 @@ class PoseEngine:
             self.post.select(ticket)
         if check:
             self.post.check_status(n)
-        return [humans_to_dicts(self.post.humans(i), W, H) for i in range(n)]
+        return [humans_to_dicts(self.post.humans(i), _of_image(W, i), _of_image(H, i)) for i in range(n)]
 
     def fetch_arrays(self, check=True, ticket=None):
         """Like fetch() but without building Python objects: per image a float32 array [k, 73] with rows
